@@ -2,7 +2,7 @@
 """Headline benchmark: edges/s of one DynConv2d forward (dilated kNN graph + EdgeConv,
 B=16 N=4096 k=20 C=64 - BASELINE.json's metric shape) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of 16 synthetic clouds
 (1,310,720 edges).  Multi-GPU: the batch dimension is sharded, every rank owns its
@@ -12,6 +12,10 @@ for everything else - NCCL's version banner, warnings).  The K timed steps are
 enqueued behind a ~2 ms spin kernel and bracketed by CUDA events: a step is ~0.25 ms
 of GPU time, so the host's first-launch latency after the synchronize would otherwise
 be several percent of a 20-step region.
+
+`--dump-outputs DIR` writes what the K-th timed step returned, DynConv2d's (16, 64, 4096, 1) fp32 output (16.8 MB),
+as DIR/y.npy once all timing is done; inputs and weights are seeded, so the file depends only on the arguments and
+on the build (`--impl reference`: its own last step, 4 clouds).
 
 `--impl reference` times the reference's CPU algorithm (the oracle port: the
 reference is pure Python/torch, there is nothing to compile into oracle/_ref) on the
@@ -57,7 +61,21 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--sustained-seconds", type=float, default=2.0, help="length of the sustained loop (N=1)")
     ap.add_argument("--no-extra", action="store_true", help="skip the multi-GPU extra blocks (N>1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step as DIR/y.npy (float32; rank 0's clouds at N>1)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(directory, arrays):
+    """{name: array} -> directory/<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be
+    compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def bind_to_gpu_numa_node(index):
@@ -274,8 +292,10 @@ def run_reference(args):
         run(x)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        run(x)
+        y = run(x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": y.numpy()})
     value = edges * args.steps / dt
     sample = ("%d of the %d clouds per step (clouds are independent), %d steps, %d threads = fastest of %s on the "
               "%d available" % (clouds, B, args.steps, threads, thread_candidates(), len(os.sched_getaffinity(0))))
@@ -421,12 +441,14 @@ def run_native(args):
             torch.cuda._sleep(4_000_000)
             beg.record()
             for i in range(args.steps):
-                mod(xs[i % N_ROTATE])
+                y = mod(xs[i % N_ROTATE])
             end.record()
             barrier()
         ms = beg.elapsed_time(end)
         knn_ms, knn_n = _native.kernel_timing_read("knn")
         _native.kernel_timing(False)
+        last_step = {"y": y.cpu().numpy()} if args.dump_outputs and rank == 0 else None
+        del y
 
         # ---- end to end: pinned host input -> device -> DynConv2d -> pinned host result -------------
         # Every step copies ITS input from pinned host memory and ITS result back, inside the timed
@@ -583,6 +605,8 @@ def run_native(args):
                                          "%d threads = fastest of %s (%d hardware threads available)"
                                          % (xc.shape[0], B, reps, dt, threads, thread_candidates(),
                                             len(os.sched_getaffinity(0)))}
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, last_step)
     json_out.write(json.dumps(out) + "\n")
     json_out.flush()
     if world > 1:

@@ -8,10 +8,9 @@ names the reference lines it follows.  The fp32 flavour issues the same ATen
 CPU ops in the same order as the reference so that it is bit-identical to the
 reference on the same host; the fp64 flavour adjudicates fp32 near-ties.
 
-Pinned by tests/test_oracle_pins.py against (a) the golden vectors under
+Pinned by tests/test_oracle_pins.py against the golden vectors under
 tests/golden/ that tests/golden/gen_golden.py produced by running the
-UNMODIFIED reference modules (oracle/ref_shims.py), and (b) the live reference
-whenever /root/reference is present.
+UNMODIFIED reference modules (oracle/ref_shims.py).
 """
 import torch
 import torch.nn.functional as F

@@ -6,10 +6,9 @@ small stand-ins for the absent packages into ``sys.modules`` and then imports
 the reference's own ``gcn_lib.dense`` / ``gcn_lib.sparse`` so that the
 reference code itself executes on CPU torch.  Used by
 
-* ``tests/golden/gen_golden.py``  - to generate the committed golden vectors,
-* ``tests/test_oracle_pins.py``   - to pin ``oracle/`` against the live
-  reference whenever ``/root/reference`` is present (it is absent on the GPU
-  box; those tests skip there and the committed vectors take over).
+* ``tests/golden/gen_golden.py`` and ``tests/golden/gen_golden_models.py`` -
+  to generate the committed golden vectors and API fixture that the tests
+  compare against; no test loads the reference itself.
 
 Third-party arithmetic restated here (none of it lives under /root/reference;
 versions are NOT pinned by the reference: deepgcn_env_install.sh:21-32 installs

@@ -169,9 +169,48 @@ def sparse_edge_cases():
          {k: v.to(torch.int32) for k, v in outs.items()})
 
 
+PIN_DENSE_SHAPES = [(1, 5, 77, 3, 2), (3, 20, 130, 7, 1), (2, 3, 64, 8, 8)]      # (B, C, N, k, dilation)
+PIN_AGGRS = ("softmax", "softmax_sg", "softmax_sum", "power", "power_sum", "add", "mean", "max")
+PIN_GRAPHS = ((4, 1), (3, 4))                                                     # (k, dilation)
+
+
+def pin_cases(dense, sparse):
+    """Small odd shapes through the reference's default-initialised modules (no randomize_norm): the dense kNN
+    matrix, DynConv2d(C, 9, k, d, conv, 'leakyrelu', 'batch') in eval, GENConv(12, 12) for every aggregator with
+    learnable t and message norm, and the sparse DilatedKnnGraph over three clouds."""
+    te = sys.modules["gcn_lib.sparse.torch_edge"]
+    g = torch.Generator().manual_seed(11)
+    ins, sd, outs = {}, {}, {}
+    for s, (B, C, N, k, d) in enumerate(PIN_DENSE_SHAPES):
+        x = torch.randn(B, C, N, 1, generator=g)
+        ins["x%d" % s] = x
+        outs["knn%d" % s] = dense.dense_knn_matrix(x, k * d).to(torch.int32)
+        for conv in ("edge", "mr"):
+            torch.manual_seed(3)
+            mod = dense.DynConv2d(C, 9, k, d, conv, "leakyrelu", "batch", True).eval()
+            with torch.no_grad():
+                outs["y%d_%s" % (s, conv)] = mod(x)
+            sd.update({"s%d_%s.%s" % (s, conv, kk): vv for kk, vv in mod.state_dict().items()})
+    ins["xs"] = torch.randn(90, 12, generator=g)
+    ins["edge_index"] = torch.randint(0, 90, (2, 500), generator=g).to(torch.int32)
+    for aggr in PIN_AGGRS:
+        torch.manual_seed(4)
+        mod = sparse.GENConv(12, 12, aggr=aggr, t=0.3, learn_t=True, p=2.0, y=0.2, msg_norm=True).eval()
+        with torch.no_grad():
+            outs["gen_" + aggr] = mod(ins["xs"], ins["edge_index"].long())
+        sd.update({"%s.%s" % (aggr, kk): vv for kk, vv in mod.state_dict().items()})
+    ins["xg"] = torch.randn(3 * 50, 6, generator=g)
+    ins["batch"] = torch.arange(3).repeat_interleave(50).to(torch.int32)
+    for k, d in PIN_GRAPHS:
+        outs["graph_k%d_d%d" % (k, d)] = te.DilatedKnnGraph(k, d)(ins["xg"], ins["batch"].long()).to(torch.int32)
+    save("pin_random_shapes", dict(dense=PIN_DENSE_SHAPES, act="leakyrelu", norm="batch", aggrs=PIN_AGGRS,
+                                   graphs=PIN_GRAPHS), ins, sd, outs)
+
+
 if __name__ == "__main__":
     torch.set_num_threads(8)
     dense, sparse = ref_shims.load_reference()
     dense_cases(dense)
     sparse_cases(sparse)
     sparse_edge_cases()
+    pin_cases(dense, sparse)

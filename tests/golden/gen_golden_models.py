@@ -174,6 +174,37 @@ def sparse_layout_convs():
          {"x": x, "edge_index": ei.to(torch.int32), "xb": xb, "batch": batch.to(torch.int32)}, sds, outs)
 
 
+API_DENSE = ("DenseDilated", "DenseDilatedKnnGraph", "DilatedKnnGraph", "MRConv2d", "EdgeConv2d", "GraphConv2d",
+             "DynConv2d", "PlainDynBlock2d", "ResDynBlock2d", "DenseDynBlock2d", "BasicConv")
+API_SPARSE = ("GENConv", "MsgNorm", "MLP")
+API_OPT = dict(n_filters=16, k=4, act="relu", norm="batch", bias=True, epsilon=0.2, stochastic=True, conv="edge",
+               n_blocks=3, block="res", in_channels=9, n_classes=13, dropout=0.3)
+
+
+def reference_api():
+    """reference_api.json: the constructor signatures of the public gcn_lib classes ([name, repr(default)] per
+    parameter) and the state_dict layout ([key, shape, dtype]) of examples/sem_seg_dense/architecture.py's
+    DenseDeepGCN at a small configuration."""
+    import inspect
+    import json
+    dense, sparse = ref_shims.load_reference()
+
+    def sig(cls):
+        return [[p.name, repr(p.default)] for p in inspect.signature(cls.__init__).parameters.values()]
+    ns = exec_reference("examples/sem_seg_dense/architecture.py", "ref_semseg")
+    torch.manual_seed(0)
+    model = ns["DenseDeepGCN"](types.SimpleNamespace(**API_OPT))
+    sigs = {n: sig(getattr(m, n)) for m, names in ((dense, API_DENSE), (sparse, API_SPARSE)) for n in names}
+    sd = [[k, list(v.shape), str(v.dtype)] for k, v in model.state_dict().items()]
+    rows = lambda lines: ",\n".join("  " + r for r in lines)      # one class / one tensor per line
+    with open(os.path.join(HERE, "reference_api.json"), "w") as fh:
+        fh.write('{"signatures": {\n%s\n },\n "dense_deep_gcn_opt": %s,\n "dense_deep_gcn_state_dict": [\n%s\n ]}\n'
+                 % (rows("%s: %s" % (json.dumps(n), json.dumps(s)) for n, s in sigs.items()), json.dumps(API_OPT),
+                    rows(json.dumps(r) for r in sd)))
+    print("wrote reference_api", len(sigs), len(sd))
+
+
 if __name__ == "__main__":
     main()
     sparse_layout_convs()
+    reference_api()

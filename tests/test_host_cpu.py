@@ -9,7 +9,6 @@ import pytest
 import torch
 
 import golden_util as gu
-from oracle import ref_shims
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -94,43 +93,29 @@ def test_sparse_state_dict_compat(name):
     assert isinstance(getattr(mod, "t", 1.0), (float, torch.nn.Parameter))
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="reference tree absent (GPU box)")
 def test_signatures_match_live_reference():
+    """Constructor signatures of the drop-in classes and the state_dict layout of a model stack built on them against
+    the reference's, as stored by gen_golden_models.py's reference_api (tests/golden/reference_api.json)."""
     import inspect
+    import json
+    from bench_models import ResGCN28
     from deep_gcns_torch_b200.gcn_lib import dense as D, sparse as S
-    rd, rs = ref_shims.load_reference()
-    pairs = [(getattr(D, n), getattr(rd, n)) for n in
-             ("DenseDilated", "DenseDilatedKnnGraph", "DilatedKnnGraph", "MRConv2d", "EdgeConv2d", "GraphConv2d",
-              "DynConv2d", "PlainDynBlock2d", "ResDynBlock2d", "DenseDynBlock2d", "BasicConv")]
-    pairs += [(getattr(S, n), getattr(rs, n)) for n in ("GENConv", "MsgNorm", "MLP")]
-    for mine, ref in pairs:
-        a, b = inspect.signature(mine.__init__), inspect.signature(ref.__init__)
-        assert [(p.name, p.default) for p in a.parameters.values()] == \
-               [(p.name, p.default) for p in b.parameters.values()], mine.__name__
-    # model stacks of the reference build on top of the drop-in classes unchanged
-    import types
-    opt = types.SimpleNamespace(n_filters=16, k=4, act="relu", norm="batch", bias=True, epsilon=0.2,
-                                stochastic=True, conv="edge", n_blocks=3, block="res", in_channels=9,
-                                n_classes=13, dropout=0.3)
-    src = open(os.path.join(ref_shims.REFERENCE_ROOT, "examples/sem_seg_dense/architecture.py")).read()
-    src = src.split('if __name__ == "__main__"')[0].replace("import __init__\n", "")
-    src = src.replace("from gcn_lib.dense import", "from deep_gcns_torch_b200.gcn_lib.dense import")
-    ns = {}
-    exec(compile(src, "architecture.py", "exec"), ns)
-    mine = ns["DenseDeepGCN"](opt)
-    import sys
-    sys.path.insert(0, os.path.join(ref_shims.REFERENCE_ROOT, "examples/sem_seg_dense"))
-    ref_src = open(os.path.join(ref_shims.REFERENCE_ROOT, "examples/sem_seg_dense/architecture.py")).read()
-    ref_src = ref_src.split('if __name__ == "__main__"')[0].replace("import __init__\n", "")
-    ns2 = {"__name__": "ref_arch"}
-    sys.path.insert(0, ref_shims.REFERENCE_ROOT)
-    try:
-        exec(compile(ref_src, "ref_architecture.py", "exec"), ns2)
-    finally:
-        sys.path.remove(ref_shims.REFERENCE_ROOT)
-    theirs = ns2["DenseDeepGCN"](opt)
-    assert list(mine.state_dict().keys()) == list(theirs.state_dict().keys())
-    mine.load_state_dict(theirs.state_dict(), strict=True)
+    with open(os.path.join(gu.GOLDEN_DIR, "reference_api.json")) as fh:
+        api = json.load(fh)
+    assert len(api["signatures"]) == 14
+    for name, ref in api["signatures"].items():
+        mine = getattr(S if name in ("GENConv", "MsgNorm", "MLP") else D, name)
+        assert [[p.name, repr(p.default)] for p in inspect.signature(mine.__init__).parameters.values()] == ref, name
+    # the reference's sem_seg_dense DenseDeepGCN, assembled from the drop-in classes (bench_models.py restates it)
+    opt = api["dense_deep_gcn_opt"]
+    assert (opt["block"], opt["conv"], opt["act"], opt["norm"], opt["bias"], opt["stochastic"], opt["epsilon"],
+            opt["dropout"]) == ("res", "edge", "relu", "batch", True, True, 0.2, 0.3)
+    mine = ResGCN28(D, opt["in_channels"], opt["n_classes"], opt["k"], opt["n_filters"], opt["n_blocks"])
+    theirs = {k: torch.zeros(shape, dtype=getattr(torch, dt.split(".")[1])) for k, shape, dt in
+              api["dense_deep_gcn_state_dict"]}
+    assert list(mine.state_dict().keys()) == list(theirs.keys())
+    assert all(v.dtype == theirs[k].dtype for k, v in mine.state_dict().items())
+    mine.load_state_dict(theirs, strict=True)
 
 
 def test_bench_line_carries_every_contract_key():
